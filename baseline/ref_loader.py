@@ -1,4 +1,4 @@
-"""Import the UNMODIFIED reference from baseline/_ref (installed by tools/install_reference.py).  Test / bench
+"""Import the UNMODIFIED reference from oracle/_ref (installed by oracle/install_reference.py).  Test / bench
 infrastructure only - nothing under must3r_b200/ imports this.
 
     ref = load_reference(curope_shim=False)     # -> namespace with .model, .engine, .Dust3rEncoder, .MUSt3R
@@ -12,7 +12,7 @@ import sys
 import types
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, "_ref")
+REF = os.path.join(os.path.dirname(HERE), "oracle", "_ref")
 _loaded = {}
 
 
@@ -26,7 +26,7 @@ def load_reference(curope_shim=False, quiet=True):
             raise RuntimeError("the reference was already imported with curope_shim=%s in this process" % _loaded["shim"])
         return _loaded["ns"]
     if not available():
-        raise ImportError("baseline/_ref is missing: run tools/install_reference.py in the build container")
+        raise ImportError("oracle/_ref is missing: run oracle/install_reference.py <checkout of the reference>")
     if REF not in sys.path:
         sys.path.insert(0, REF)
     stubs = os.path.join(HERE, "stubs")

@@ -2,6 +2,7 @@
 """bench.py — views/sec of the MUSt3R multi-view inference hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3|c2|c4|c5] [--dtype bf16|fp16] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one whole job of a configuration of BASELINE.json (SURVEY.md §8d), on synthetic views and random-init
 ViT-L encoder / ViT-B memory decoder:
@@ -16,10 +17,12 @@ ViT-L encoder / ViT-B memory decoder:
 
 Prints ONE JSON line (rank 0).  `value` = device-timed views/s with inputs resident in HBM; `e2e` = the same job through
 the public engine API from pinned HOST images to HOST results (H2D / D2H inside the timed region); `parity` = rel-L2 of
-the timed job's own outputs against the UNMODIFIED reference (baseline/_ref) run in fp32 on the same GPU, for fp16 and
+the timed job's own outputs against the UNMODIFIED reference (oracle/_ref) run in fp32 on the same GPU, for fp16 and
 bf16 operands; `roofline` = per-kernel-category achieved TFLOP/s vs the measured bf16 peak; `cpu_baseline` = the
 unmodified reference's engine on this box's host cores on a bounded sample; `records` = the other configurations.
-`--impl reference` times that CPU path alone.
+`--impl reference` times that CPU path alone.  `--dump-outputs DIR` writes what the last timed step returned (rank 0's
+views) as DIR/<name>.npy; inputs and weights are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -72,6 +75,27 @@ def sharded_schedule(counts):
         m_cur += part
     tot = sum(counts)
     return upd, [(tot, tot)]
+
+
+DUMP_BUDGET = 64 << 20
+
+
+def dump_outputs(out, path, budget=DUMP_BUDGET):
+    """Write the per-view result dicts a caller of the timed path receives, stacked over views, as <path>/<name>.npy in
+    float32.  When the arrays exceed `budget` bytes in all, each keeps a fixed sample of its flattened elements (sorted
+    indices drawn by numpy's default_rng(0), a share of the budget proportional to its size), so the files of two runs
+    with the same arguments line up element for element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: torch.stack([d[k] for d in out]).float() for k in out[0]}
+    total = sum(a.numel() for a in arrays.values()) * 4
+    for k, a in arrays.items():
+        if total > budget:
+            n = a.numel()
+            idx = np.unique(np.random.default_rng(0).integers(0, n, size=n * budget // total))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(path, f"{k}.npy"), a.cpu().numpy())
+    return sorted(arrays)
 
 
 def effective_cores():
@@ -160,7 +184,7 @@ def reference_available():
 
 
 def build_reference(size, device, curope_shim):
-    """The UNMODIFIED reference's classes (baseline/_ref, installed by tools/install_reference.py) with the synthetic weights."""
+    """The UNMODIFIED reference's classes (oracle/_ref, installed by oracle/install_reference.py) with the synthetic weights."""
     from baseline import ref_loader
     from must3r_b200 import synthetic as syn
     ref = ref_loader.load_reference(curope_shim=curope_shim)
@@ -174,7 +198,7 @@ def build_reference(size, device, curope_shim):
 def cpu_reference_job(cfg, n_views, threads):
     """The reference's own engine on host cores (must3r/engine/inference.py:370 inference_multi_ar, SDPA branch, PyTorch RoPE
     fallback, fp32): the first `n_views` views of the configuration = encoder + 2-view init + (n-2) one-view updates +
-    render of the n views + activation.  Falls back to the oracle port (kind "port") when baseline/_ref is absent."""
+    render of the n views + activation.  Falls back to the oracle port (kind "port") when oracle/_ref is absent."""
     from must3r_b200 import synthetic as syn
     torch.set_num_threads(threads)
     H, W, size = cfg["H"], cfg["W"], cfg["size"]
@@ -217,7 +241,7 @@ def run_reference_arm(args, rank, world):
         job()
     dt = (time.perf_counter() - t0) / args.steps
     v = n / dt
-    what = "unmodified reference (baseline/_ref, must3r.engine.inference_multi_ar, fp32, SDPA, RoPE fallback)" if kind == "reference" else "oracle port (baseline/_ref missing)"
+    what = "unmodified reference (oracle/_ref, must3r.engine.inference_multi_ar, fp32, SDPA, RoPE fallback)" if kind == "reference" else "oracle port (oracle/_ref missing)"
     sample = f"{n} of the {cfg['V']} views per step ({cfg['H']}x{cfg['W']}: encoder + 2-view init + {n - 2} one-view update(s) + render {n} + activation), {what}"
     print(json.dumps({
         "impl": "reference", "metric": "views/sec at 512x384 (ViT-L enc / ViT-B dec)", "value": v, "unit": "views/s",
@@ -244,10 +268,14 @@ def main():
     ap.add_argument("--no-records", action="store_true", help="skip the extra configurations (records)")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--stream-frames", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     ap.add_argument("--encoder-mode", default="precomputed", choices=["engine", "precomputed"],
                     help="precomputed (default): engine.encoder_multi_ar over all views first, then the decoder chain (features handed to "
                          "the engine); engine: encoder_precomputed_features=None, the engine encodes the missing views itself (up front, batched)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -390,7 +418,7 @@ def main():
         """rel-L2 of the job's rendered outputs (raw head, pts3d, conf) vs the unmodified reference run in fp32 on this GPU
         (TF32 off, its RoPE served by must3r_b200.compat.curope), for fp16 and bf16 operands.  Single-GPU chain configs."""
         if args.no_parity or not reference_available():
-            return {"unavailable": "baseline/_ref missing" if not args.no_parity else "--no-parity"}
+            return {"unavailable": "oracle/_ref missing" if not args.no_parity else "--no-parity"}
         V, H, W = cfg["V"], cfg["H"], cfg["W"]
         torch.backends.cuda.matmul.allow_tf32 = False
         torch.backends.cudnn.allow_tf32 = False
@@ -409,7 +437,7 @@ def main():
             r_post = ref.engine.postprocess(r_raw, ref.model.ActivationType.NORM_EXP)
         del renc, rdec
         rel = lambda a, b: float((a.double() - b.double()).norm() / b.double().norm())  # noqa: E731
-        out = {"against": "unmodified reference (baseline/_ref) fp32 on this GPU, TF32 off, same schedule through its own engine",
+        out = {"against": "unmodified reference (oracle/_ref) fp32 on this GPU, TF32 off, same schedule through its own engine",
                "views": V, "reference_gpu_ms_per_job": round(t_ref * 1e3, 1)}
         for dt in (torch.float16, torch.bfloat16):
             set_precision(dt)
@@ -428,7 +456,7 @@ def main():
         (fp32, rank 0's GPU): rounds of one-view updates against the memory of the previous rounds, tokens appended in rank
         order, then render (tests/test_sharded_cpu.py composes the oracle the same way)."""
         if args.no_parity or not reference_available():
-            return {"unavailable": "baseline/_ref missing" if not args.no_parity else "--no-parity"}
+            return {"unavailable": "oracle/_ref missing" if not args.no_parity else "--no-parity"}
         counts = meta["counts"]
         raw = lambda pm: {"raw": pm}  # noqa: E731
         res = {}
@@ -484,9 +512,16 @@ def main():
         job()
     barrier()
     launches0 = lib.m3r_launch_count()
-    ms = timed(job, args.steps, 0, sampler=clk)
+    last = {}
+
+    def job_keep_output():
+        last["out"] = job()
+    ms = timed(job_keep_output if args.dump_outputs else job, args.steps, 0, sampler=clk)
     launches = (lib.m3r_launch_count() - launches0) // args.steps
     value = meta["views"] / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last["out"], args.dump_outputs)
+    last.clear()
 
     # ---- end to end: pinned host images -> host results (H2D / D2H inside the timed region)
     out = None

@@ -266,6 +266,40 @@ def engine_golden():
     print("engine.npz", len(out), "arrays")
 
 
+def keyframes_golden():
+    """SLAM keyframe overlap scores (must3r/slam/model.py get_overlap_score, choose_keyframe_from_overlap) with the
+    reference's scipy searchers (must3r/slam/nns.py), and its quadrant ids (must3r/slam/tools.py get_quadrant_id), on the
+    seeded frames of tests/helpers.py -> tests/golden/keyframes.npz."""
+    import importlib
+    sys.path.insert(0, os.path.dirname(HERE))
+    import helpers as h
+    nns, model = importlib.import_module("must3r.slam.nns"), importlib.import_module("must3r.slam.model")
+    tools = importlib.import_module("must3r.slam.tools")
+    out = {}
+    cam = torch.tensor(h.KEYFRAME_CAM)
+    for method in h.KEYFRAME_METHODS:
+        for mode in ("nn", "nn-norm"):
+            tree = nns.get_searcher(method)
+            for seed, shift in h.KEYFRAME_DB:
+                fr = h.keyframe_frame(seed, shift=shift)
+                tree.add_pts(fr["pts3d"][0, 0, ::2, ::2][fr["conf"][0, 0, ::2, ::2] > 1.5], cam_center=cam)
+            for seed, shift in h.KEYFRAME_QUERIES:
+                s = model.get_overlap_score(h.keyframe_frame(seed, shift=shift), tree, cam, mode=mode, kf_x_subsamp=2,
+                                            min_conf_keyframe=1.5, percentile=70)
+                out[f"{method}.{mode}.{seed}.score"] = np.float64(s)
+                out[f"{method}.{mode}.{seed}.choice"] = np.bool_(model.choose_keyframe_from_overlap(s, 0.1, mode))
+        s = model.get_overlap_score(h.keyframe_frame(60), nns.get_searcher(method), cam, mode="nn", kf_x_subsamp=2)
+        out[f"{method}.empty.score"] = np.float64(s)
+    fr = h.keyframe_frame(70)
+    for mode in ("meanconf", "medianconf"):
+        out[f"{mode}.score"] = np.float64(model.get_overlap_score(fr, None, None, mode=mode))
+    rays = torch.randn(4000, 3, generator=torch.Generator().manual_seed(3))
+    for div in (2, 4):
+        out[f"quadrant{div}"] = np.asarray(tools.get_quadrant_id(rays.clone().numpy(), quadrant_divider=div)).astype(np.int8)
+    np.savez_compressed(os.path.join(HERE, "keyframes.npz"), **out)
+    print("keyframes.npz", len(out), "arrays")
+
+
 def model_args_golden():
     """Constructor-string rewrites of load_model (must3r/model/__init__.py:53-108) -> tests/golden/model_args.json."""
     import json
@@ -295,3 +329,5 @@ if __name__ == "__main__":
         full_model_golden()
     if "chain" in which:
         chain_golden()
+    if "keyframes" in which:
+        keyframes_golden()

@@ -41,6 +41,22 @@ def digest(t, max_elems=4096):  # same sampling as tests/golden/make_golden.py
                            np.array([f.mean(), f.std(), f.abs().sum() / f.numel()], dtype=np.float32)])
 
 
+def keyframe_frame(seed, H=48, W=64, shift=0.0):
+    """A random postprocessed frame (pts3d, pts3d_local with positive depth, conf >= 1) for the keyframe overlap tests."""
+    g = torch.Generator().manual_seed(seed)
+    pts = torch.randn(1, 1, H, W, 3, generator=g) * 2.0 + shift
+    loc = pts.clone()
+    loc[..., 2] = loc[..., 2].abs() + 1.0
+    conf = 1.0 + torch.rand(1, 1, H, W, generator=g) * 3.0
+    return {"pts3d": pts, "pts3d_local": loc, "conf": conf}
+
+
+KEYFRAME_METHODS = ["kdtree-scipy", "quadrant_x2-kdtree-scipy", "quadrant_x4-kdtree-scipy"]
+KEYFRAME_DB = [(10 + i, 0.5 * i) for i in range(3)]      # (seed, shift) of the three keyframes stored in the database
+KEYFRAME_QUERIES = [(50, 0.2), (51, 3.0)]                 # an overlapping and a far-away frame
+KEYFRAME_CAM = (0.1, -0.2, 0.3)
+
+
 def rel(a, b):
     a = torch.as_tensor(np.asarray(a)).double()
     b = torch.as_tensor(np.asarray(b)).double()

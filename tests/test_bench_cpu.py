@@ -34,11 +34,31 @@ def test_split_and_schedules():
     assert abs(f - want) / want < 1e-12 and 31.0e12 < f < 32.0e12
 
 
+def test_dump_outputs_whole_or_fixed_sample(tmp_path):
+    """--dump-outputs: the per-view result dicts stacked over views, float32; within the budget the arrays are written
+    whole, above it every file holds the same sample of its array on every run and the files stay within the budget."""
+    import numpy as np
+    import torch
+    g = torch.Generator().manual_seed(0)
+    out = [{"pts3d": torch.randn(4, 5, 3, generator=g), "conf": torch.rand(4, 5, generator=g, dtype=torch.float64)} for _ in range(3)]
+    full = {k: torch.stack([d[k] for d in out]).float().numpy() for k in ("pts3d", "conf")}
+    assert bench.dump_outputs(out, str(tmp_path / "whole")) == ["conf", "pts3d"]
+    for k, want in full.items():
+        got = np.load(tmp_path / "whole" / f"{k}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, want)
+    for run in ("a", "b"):
+        bench.dump_outputs(out, str(tmp_path / run), budget=200)
+    a = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in full}
+    assert sum(v.nbytes for v in a.values()) <= 200 and all(v.size > 0 and v.dtype == np.float32 for v in a.values())
+    for k, v in a.items():
+        assert np.array_equal(v, np.load(tmp_path / "b" / f"{k}.npy")) and np.isin(v, full[k]).all()
+
+
 @pytest.mark.timeout(600)
 def test_reference_arm_prints_the_contract_line():
     from baseline import ref_loader
     if not ref_loader.available():
-        pytest.skip("baseline/_ref not installed")
+        pytest.skip("the reference is not installed under oracle/_ref")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--config", "c2", "--steps", "1",
                           "--warmup", "1", "--cpu-views", "2"], capture_output=True, text=True, timeout=500)
     assert out.returncode == 0, out.stderr[-2000:]

@@ -1,6 +1,6 @@
 """SLAM keyframe overlap score on the GPU (must3r_b200/engine/keyframes.py) against the UNMODIFIED reference's own
-functions (baseline/_ref: must3r/slam/model.py:62-91 get_overlap_score, must3r/slam/nns.py searchers on scipy KD-trees)."""
-import importlib
+functions (must3r/slam/model.py:62-91 get_overlap_score, must3r/slam/nns.py searchers on scipy KD-trees), whose outputs
+on the same seeded frames are stored in tests/golden/keyframes.npz (tests/golden/make_golden.py keyframes)."""
 import os
 import sys
 
@@ -10,24 +10,10 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from baseline import ref_loader  # noqa: E402
+from helpers import KEYFRAME_CAM, KEYFRAME_DB, KEYFRAME_METHODS, KEYFRAME_QUERIES, keyframe_frame, load_golden  # noqa: E402
 from must3r_b200.engine import keyframes as kf  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="baseline/_ref not installed")]
-
-
-def _ref():
-    ref_loader.load_reference(curope_shim=True)       # one RoPE choice per process: every GPU test loads the reference with the shim
-    return importlib.import_module("must3r.slam.nns"), importlib.import_module("must3r.slam.model")
-
-
-def _frame(seed, H=48, W=64, shift=0.0):
-    g = torch.Generator().manual_seed(seed)
-    pts = torch.randn(1, 1, H, W, 3, generator=g) * 2.0 + shift
-    loc = pts.clone()
-    loc[..., 2] = loc[..., 2].abs() + 1.0
-    conf = 1.0 + torch.rand(1, 1, H, W, generator=g) * 3.0
-    return {"pts3d": pts, "pts3d_local": loc, "conf": conf}
+pytestmark = pytest.mark.gpu
 
 
 def test_nn_min_dist_matches_brute_force_and_kdtree():
@@ -40,40 +26,38 @@ def test_nn_min_dist_matches_brute_force_and_kdtree():
     assert torch.isinf(kf.nn_min_dist(q.cuda(), torch.zeros(0, 3).cuda())).all()
 
 
-@pytest.mark.parametrize("method", ["kdtree-scipy", "quadrant_x2-kdtree-scipy", "quadrant_x4-kdtree-scipy"])
+@pytest.mark.parametrize("method", KEYFRAME_METHODS)
 @pytest.mark.parametrize("mode", ["nn", "nn-norm"])
 def test_overlap_score_matches_reference(method, mode):
-    nns, model = _ref()
-    tree_ref, tree = nns.get_searcher(method), kf.get_searcher(method)
-    cam = torch.tensor([0.1, -0.2, 0.3])
-    for i in range(3):                                   # three keyframes in the database
-        fr = _frame(10 + i, shift=0.5 * i)
+    g = load_golden("keyframes.npz")
+    tree = kf.get_searcher(method)
+    cam = torch.tensor(KEYFRAME_CAM)
+    for seed, shift in KEYFRAME_DB:                      # three keyframes in the database
+        fr = keyframe_frame(seed, shift=shift)
         sel = fr["pts3d"][0, 0, ::2, ::2][fr["conf"][0, 0, ::2, ::2] > 1.5]
-        tree_ref.add_pts(sel, cam_center=cam)
         tree.add_pts(sel.cuda(), cam_center=cam.cuda())
-    for seed, shift in ((50, 0.2), (51, 3.0)):           # an overlapping and a far-away frame
-        fr = _frame(seed, shift=shift)
-        want = model.get_overlap_score(fr, tree_ref, cam, mode=mode, kf_x_subsamp=2, min_conf_keyframe=1.5, percentile=70)
+    for seed, shift in KEYFRAME_QUERIES:                 # an overlapping and a far-away frame
+        fr = keyframe_frame(seed, shift=shift)
+        want = float(g[f"{method}.{mode}.{seed}.score"])
         got = kf.get_overlap_score({k: v.cuda() for k, v in fr.items()}, tree, cam.cuda(), mode=mode, kf_x_subsamp=2,
                                    min_conf_keyframe=1.5, percentile=70)
         assert abs(got - want) <= 2e-5 * max(1.0, abs(want)), (method, mode, got, want)
-        assert kf.choose_keyframe_from_overlap(got, 0.1, mode) == model.choose_keyframe_from_overlap(want, 0.1, mode)
+        assert kf.choose_keyframe_from_overlap(got, 0.1, mode) == bool(g[f"{method}.{mode}.{seed}.choice"])
     empty = kf.get_searcher(method)                      # nothing stored yet: every distance is "infinite"
-    fr = _frame(60)
-    want = model.get_overlap_score(fr, nns.get_searcher(method), cam, mode="nn", kf_x_subsamp=2)
+    fr = keyframe_frame(60)
+    want = float(g[f"{method}.empty.score"])
     got = kf.get_overlap_score({k: v.cuda() for k, v in fr.items()}, empty, cam.cuda(), mode="nn", kf_x_subsamp=2)
-    assert got == pytest.approx(float(want), rel=1e-6) or (got > 1e30 and want > 1e30)
+    assert got == pytest.approx(want, rel=1e-6) or (got > 1e30 and want > 1e30)
 
 
 def test_conf_modes_and_quadrants():
-    nns, model = _ref()
-    tools = importlib.import_module("must3r.slam.tools")
-    fr = _frame(70)
+    g = load_golden("keyframes.npz")
+    fr = keyframe_frame(70)
     for mode in ("meanconf", "medianconf"):
         assert float(kf.get_overlap_score({k: v.cuda() for k, v in fr.items()}, None, None, mode=mode)) == pytest.approx(
-            float(model.get_overlap_score(fr, None, None, mode=mode)), rel=1e-6)
+            float(g[f"{mode}.score"]), rel=1e-6)
     rays = torch.randn(4000, 3, generator=torch.Generator().manual_seed(3))
     for div in (2, 4):
-        want = tools.get_quadrant_id(rays.clone().numpy(), quadrant_divider=div)
+        want = g[f"quadrant{div}"]
         got = kf.get_quadrant_id(rays.cuda(), div).cpu().numpy()
         assert (got != want).mean() < 1e-3                # bin edges: fp32 vs fp64 trig may differ on a handful of rays

@@ -112,7 +112,12 @@ def test_gloo_matches_composed_oracle(world, counts):
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
-    mem, renders = _composed_expected(world, counts)
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)              # as in the workers: how a CPU GEMM splits its sums depends on the thread count
+    try:
+        mem, renders = _composed_expected(world, counts)
+    finally:
+        torch.set_num_threads(threads)
     for r in range(world):
         outs, mem_vals, labels = got[r]
         assert torch.equal(labels, mem[1])                                   # identical memory on every rank

@@ -2,7 +2,7 @@
 device-side flag barrier, or NCCL all-gather with M3R_FUSED_GATHER=0) must
   (1) reproduce, bit for bit, the same schedule composed from single-process CUDA decoder calls, with identical memory on
       all ranks - also on a second call that reuses the cached peer arena, and with a ragged split of the views;
-  (2) match the schedule composed from single-process calls of the UNMODIFIED reference (baseline/_ref, fp32 on this GPU)
+  (2) match the schedule composed from single-process calls of the UNMODIFIED reference (oracle/_ref, fp32 on this GPU)
       at 512x384 within the fp16-operand tolerance (SURVEY.md 8e oracle).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/check_sharded.py"""
 import os, sys
@@ -104,7 +104,7 @@ def run_case(tag, size, H, W, depth_e, depth_d, counts, dtype, calls=1, vs_refer
             msg += f"; vs composed UNMODIFIED reference (fp32): render {e_ref:.2e}, last-level memory {e_mem:.2e} (gate {gate:.1e})"
             ok = ok and e_ref < gate and e_mem < 1.3 * gate
         else:
-            msg += "; baseline/_ref missing: reference composition skipped"
+            msg += "; oracle/_ref missing: reference composition skipped"
     print(msg, flush=True)
     ok_all = ok_all and ok
 
